@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- images/s of the ctdet heat-map decode hot path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One step = one ctdet_decode pass (3x3 peak-NMS + top-K + wh/reg gather + box assembly)
@@ -14,6 +14,10 @@ over ranks); `e2e` = same metric through the public API with pinned HOST buffers
 H2D of the heat/wh/reg batch and the D2H of the detections inside the timed region;
 `roofline` = algorithmic bytes / device time against MEASURED_PEAKS.json;
 `cpu_baseline` = the CPU port of the reference path on a bounded sample.
+
+--dump-outputs DIR writes the detections of the last timed step, [64, K, 6] float32, to DIR/dets.npy
+(DIR/dets.rank<r>.npy per rank when N > 1).  The inputs are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 import argparse
 import json
@@ -26,6 +30,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (it may be read-only)
 
 METRIC = "images/sec ctdet 512x512->128x128x80 heatmap decode K=100"
 UNIT = "images/s"
@@ -242,7 +247,14 @@ def main():
                     help="pin the rank to its GPU's NUMA node before allocating (default: only when world > 1)")
     ap.add_argument("--no-bind-numa", dest="bind_numa", action="store_false")
     ap.add_argument("--no-secondary", action="store_true", help="skip the per-kernel secondary measurements (N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the detections of the last timed step to DIR/dets.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        # the reference arm decodes a host-timed sample of the batch whose size varies from run to run
+        ap.error("--dump-outputs needs --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -301,6 +313,11 @@ def main():
     sampler.force_sample()
     launches = CL.launch_count() - l0
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        name = "dets.npy" if world == 1 else "dets.rank%d.npy" % rank
+        np.save(os.path.join(args.dump_outputs, name), dets.float().cpu().numpy())
     sampler.stop_flag = True
     sampler.join(timeout=2)
     t = torch.tensor([ms], device=dev)

@@ -8,7 +8,7 @@ try:
     from . import _C
 except ImportError as e:  # pragma: no cover - exercised only on a broken install
     raise ImportError(
-        "centernet_b200: the CUDA extension is not built (%s). Run `python -m centernet_b200.build` "
+        "centernet_b200: the CUDA extension is not built (%s). Run `python centernet_b200/build.py` "
         "(needs nvcc, targets sm_100a). There is no CPU fallback." % (e,)) from e
 
 

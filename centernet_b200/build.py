@@ -3,7 +3,7 @@
   centernet_b200/lib/libcenternet_b200.so   <- nvcc, every csrc/*.cu   (the C ABI)
   centernet_b200/_C<ext>.so                 <- g++,  csrc/pybind.cpp    (thin binding)
 
-Run as ``python -m centernet_b200.build`` (add ``--force`` to rebuild).  nvcc
+Run as ``python centernet_b200/build.py`` (add ``--force`` to rebuild).  nvcc
 cross-compiles without a GPU, so this also runs in the CPU-only build container.
 """
 import glob

@@ -15,5 +15,5 @@ def pytest_configure(config):
 @pytest.fixture(scope="session", autouse=True)
 def _built_extension():
     """Make sure the in-tree extension exists (nvcc cross-compiles without a GPU)."""
-    from centernet_b200.build import build
-    build()
+    import __graft_entry__
+    __graft_entry__._builder().build()

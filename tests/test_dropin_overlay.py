@@ -1,7 +1,8 @@
 """A17 / drop-in boundary: dropin/ overlaid on a temp copy of the reference's src/ -- the reference's own
 callers (detectors/*.py, trains/*.py, models/model.py, the DCN networks) import and build unchanged on top
-of centernet_b200.  CPU, build container only (needs /root/reference; skipped on the GPU box).  The run
-happens in a subprocess so the stub modules and sys.path edits stay out of the test process."""
+of centernet_b200.  CPU; needs a checkout of the original CenterNet, whose src/ directory CENTERNET_SRC names
+(skipped without it).  The run happens in a subprocess so the stub modules and sys.path edits stay out of the
+test process."""
 import os
 import shutil
 import subprocess
@@ -10,7 +11,7 @@ import textwrap
 
 import pytest
 
-REF_SRC = "/root/reference/src"
+REF_SRC = os.environ.get("CENTERNET_SRC", "")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 SCRIPT = textwrap.dedent('''
@@ -91,7 +92,7 @@ SCRIPT = textwrap.dedent('''
 ''')
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="needs /root/reference (build container only)")
+@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="set CENTERNET_SRC to the src/ of a CenterNet checkout")
 def test_reference_callers_import_on_the_overlay(tmp_path):
     src = tmp_path / "src"
     shutil.copytree(REF_SRC, src)

@@ -52,20 +52,14 @@ def test_oracle_soft_nms_39_and_merge():
 
 
 def test_reference_nms_module_if_built():
-    """Where oracle/_ref holds the compiled reference (build container, GPU box), the oracle is also checked live
-    against it on fresh random lists."""
-    from oracle import build_ref
-    ref = build_ref.load_nms()
-    if ref is None:
-        pytest.skip("oracle/_ref nms module not built")
-    rng = np.random.default_rng(5)
-    for method, Nt in ((2, 0.5), (1, 0.3), (0, 0.4)):
-        x = rng.uniform(0, 200, 70); y = rng.uniform(0, 200, 70)
-        b = np.stack([x, y, x + rng.uniform(10, 90, 70), y + rng.uniform(10, 90, 70), rng.uniform(0, 1, 70)], 1).astype(np.float32)
-        a1, a2 = b.copy(), b.copy()
-        keep = ref.soft_nms(a1, Nt=Nt, method=method)
-        assert O.soft_nms(a2, Nt=Nt, method=method) == len(keep)
-        np.testing.assert_array_equal(a1, a2)
+    """The oracle against the compiled reference soft_nms on three random 70-box lists (gaussian, linear, hard):
+    tests/golden/nms_lists.npz holds what the reference module returned for them (make_golden_nms.py)."""
+    g = golden("nms_lists")
+    for i in range(3):
+        method, Nt = g["cfg%d" % i]
+        a = g["in%d" % i].copy()
+        assert O.soft_nms(a, Nt=float(Nt), method=int(method)) == int(g["n%d" % i])
+        np.testing.assert_array_equal(a, g["out%d" % i])
 
 
 # --------------------------------------------------------------------------- GPU: the CUDA path

@@ -1,6 +1,6 @@
 """Tuning aid: per-CTA cycle breakdown of k_select_hot on the bench workload.  Needs a library built with the
 statistics compiled in (they are NOT in the production build):
-    CNB_NVCC_DEFINES=-DCNB_SELECT_STATS python -m centernet_b200.build --force && python tools/select_stats.py"""
+    CNB_NVCC_DEFINES=-DCNB_SELECT_STATS python centernet_b200/build.py --force && python tools/select_stats.py"""
 import ctypes
 import os
 import sys
