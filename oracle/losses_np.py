@@ -31,6 +31,20 @@ def neg_loss(pred, gt):
 
 def neg_loss_grad(pred, gt):
     """d _neg_loss / d pred (analytic; for checking the fused backward)."""
+    return _neg_loss_grad64(pred, gt).astype(F32)
+
+
+def neg_loss_grad_logits(s32, gt):
+    """d (_sigmoid + _neg_loss) / d logit in float64.  s32 is the fp32 sigmoid of the logits (what torch's
+    sigmoid returns); torch.clamp's backward passes the gradient only where 1e-4 <= s32 <= 1-1e-4 (inclusive)."""
+    s32 = np.asarray(s32, F32)
+    lo, hi = F32(1e-4), F32(1 - 1e-4)
+    s = s32.astype(np.float64)
+    chain = np.where((s32 >= lo) & (s32 <= hi), s * (1 - s), 0.0)
+    return _neg_loss_grad64(np.clip(s32, lo, hi), gt) * chain
+
+
+def _neg_loss_grad64(pred, gt):
     pred = np.asarray(pred, np.float64); gt = np.asarray(gt, np.float64)
     pos = (gt == 1); neg = (gt < 1)
     num_pos = pos.sum()
@@ -40,8 +54,7 @@ def neg_loss_grad(pred, gt):
     # d/dp [log(1-p) p^2 w] = w(2p log(1-p) - p^2/(1-p))
     w = (1 - gt) ** 4
     g[neg] = (w * (2 * pred * np.log(1 - pred) - pred ** 2 / (1 - pred)))[neg]
-    g = -g / (num_pos if num_pos > 0 else 1.0)
-    return g.astype(F32)
+    return -g / (num_pos if num_pos > 0 else 1.0)
 
 
 def _gather_pred(output, ind):

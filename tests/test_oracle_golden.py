@@ -88,6 +88,25 @@ def test_losses():
     loss0, npos0 = losses_np.neg_loss(g["pred"], np.minimum(g["gt"], 0.5))
     assert npos0 == 0
     np.testing.assert_allclose(loss0, g["neg_loss_nopos"], rtol=1e-5)
+    # gradient w.r.t. the logit: float64 autograd of _sigmoid (clamp(sigmoid(x))) + _neg_loss.  The logits x4 put
+    # part of the map outside the clamp, where the gradient must be exactly 0.
+    import torch
+    gt = torch.from_numpy(g["gt"]).double()
+    for scale in (1.0, 4.0):
+        x32 = g["logits"] * np.float32(scale)
+        x = torch.from_numpy(x32).double().requires_grad_(True)
+        pr = torch.clamp(torch.sigmoid(x), 1e-4, 1 - 1e-4)
+        pos, neg = (gt == 1).double(), (gt < 1).double()
+        ref = -((torch.log(pr) * (1 - pr) ** 2 * pos).sum()
+                + (torch.log(1 - pr) * pr ** 2 * (1 - gt) ** 4 * neg).sum()) / pos.sum()
+        ref.backward()
+        want = x.grad.numpy()
+        s32 = (1 / (1 + np.exp(-x32.astype(np.float64)))).astype(np.float32)
+        got = losses_np.neg_loss_grad_logits(s32, g["gt"])
+        assert got.dtype == np.float64
+        np.testing.assert_array_equal(got == 0, want == 0)
+        assert (want == 0).any() == (scale > 1)
+        np.testing.assert_allclose(got, want, rtol=1e-5, atol=1e-6 * np.abs(want).max())
     a = (g["output"], g["mask"], g["ind"], g["target"])
     np.testing.assert_allclose(losses_np.reg_l1_loss(*a), g["reg_l1"], rtol=1e-5)
     np.testing.assert_allclose(losses_np.reg_loss(*a), g["reg_sl1"], rtol=1e-5)

@@ -133,7 +133,7 @@ def test_golden_splat_and_fused_focal():
     C, H, W = int(g["C"]), int(g["H"]), int(g["W"])
     cls, cx, cy, rad, val = dev(g["obj_cls"], g["obj_cx"], g["obj_cy"], g["obj_radius"], g["obj_valid"])
     hm = L.splat_gaussian(cls, cx, cy, rad, val, C, H, W)
-    np.testing.assert_allclose(hm.cpu().numpy(), g["hm"], rtol=0, atol=1e-7)
+    np.testing.assert_array_equal(hm.cpu().numpy(), g["hm"])
     assert np.array_equal(hm.cpu().numpy() == 1.0, g["hm"] == 1.0)           # identical positive set
     # fused splat+focal == focal on the dense reference target
     B = cls.shape[0]
@@ -159,7 +159,7 @@ def test_focal_full_size_linearity():
     val = torch.ones(B, M, dtype=torch.uint8, device="cuda")
     gt = L.splat_gaussian(cls, cx, cy, rad, val, C, H, W)
     want = image_np.splat_objects(*[t.cpu().numpy() for t in (cls, cx, cy, rad, val)], C, H, W)
-    np.testing.assert_allclose(gt.cpu().numpy(), want, rtol=0, atol=1e-7)
+    np.testing.assert_array_equal(gt.cpu().numpy(), want)
     full = L._neg_loss(pred, gt)
     fused = L.FocalSplatLoss()(pred, cls, cx, cy, rad, val)
     np.testing.assert_allclose(full.item(), fused.item(), rtol=1e-6)
